@@ -1,8 +1,12 @@
 #!/usr/bin/env python
 """bench.py — the MPPI command() hot path on B200, BASELINE.json's metric.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl engine|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl engine|reference] [--workload NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+Every timed loop (per-step events, back-to-back, e2e) runs exactly K steps.  `--dump-outputs DIR` writes what the last
+timed command() handed its caller (see `command_outputs`) as DIR/<name>.npy; the inputs are seeded, so two builds run
+with the same arguments can be compared output for output.
 
 One "step" = one `command()` (shift + sample K x T noise + T-step rollout + softmin reweight + nominal update).
 Workloads (BASELINE.json `configs`; the default is configs[1], the north star):
@@ -262,12 +266,9 @@ def run_reference(args, wl):
     cores = pick_cpu_threads(wl, K)
     arm = CpuArm(wl, K)
     n_warm = max(min(args.warmup, 5), 1)
-    t0 = time.perf_counter()
     for _ in range(n_warm):
         arm.step()
-    t_step = (time.perf_counter() - t0) / n_warm
-    # bounded: the timed region stays under ~2 minutes whatever --steps asks for (at least 10 commands)
-    steps = max(min(args.steps, int(120.0 / t_step)), min(args.steps, 10))
+    steps = args.steps
     t0 = time.perf_counter()
     for _ in range(steps):
         arm.step()
@@ -307,6 +308,18 @@ def make_engine(eng, wl, K_global, dev, pg, exchange, seed=1234):
     m = eng.LinearPoint.toy2d_nav()
     return eng.KMPPI(m.dynamics, m.running_cost, 2, torch.eye(2) * wl["sigma"], terminal_state_cost=m.terminal_cost,
                      u_max=torch.tensor([1.0, 1.0]), num_support_pts=wl["S"], kernel=eng.RBFKernel(sigma=wl["rbf_sigma"]), **kw)
+
+
+def command_outputs(ctrl, action):
+    """What one command() hands its caller, copied to the host: the returned action, the updated nominal sequence U,
+    the per-sample total cost (this rank's shard of the K samples) and, for KMPPI, the updated control points."""
+    out = {"action": action, "U": ctrl.U, "cost_total": ctrl.cost_total}
+    if hasattr(ctrl, "theta"):
+        out["theta"] = ctrl.theta
+    out = {k: v.detach().to("cpu", torch.float64 if v.dtype == torch.float64 else torch.float32).numpy()
+           for k, v in out.items()}
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20
+    return out
 
 
 def run_engine(args, wl):
@@ -388,13 +401,18 @@ def run_engine(args, wl):
         for e0, e1 in evs:
             flush.zero_()
             e0.record(stream)
-            ctrl.command(x_dev)
+            action = ctrl.command(x_dev)
             e1.record(stream)
         torch.cuda.synchronize()
         step_ms += [e0.elapsed_time(e1) for e0, e1 in evs]
         done += n
     barrier()
     t_end = time.time()
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in command_outputs(ctrl, action).items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     stats = trimmed_stats(step_ms)
     # max over ranks of the per-rank figures (every rank times the same K steps)
     agg = torch.tensor([stats["trimmed_mean"], stats["mean"], stats["median"], stats["min"]], dtype=torch.float64, device=dev)
@@ -406,7 +424,7 @@ def run_engine(args, wl):
 
     # ---- back-to-back launches (no flush): the steady-state command rate ---------------------------
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    nb2b = max(min(args.steps, 2000), 200)
+    nb2b = args.steps
     barrier()
     e0.record(stream)
     for _ in range(nb2b):
@@ -423,7 +441,7 @@ def run_engine(args, wl):
     for _ in range(20):
         ctrl.command_host(x_host)
     barrier()
-    n_e2e = max(args.steps, 2000) if K_gpu * T < 4_000_000 else max(min(args.steps, 2000), 300)
+    n_e2e = args.steps
     t0 = time.perf_counter()
     for _ in range(n_e2e):
         a_host = ctrl.command_host(x_host)
@@ -574,10 +592,16 @@ def main():
     ap.add_argument("--no-resident", action="store_true",
                     help="e2e on the launch route only (default at N=1: also time the host loop on a resident grid, "
                          "csrc/mppi_resident.cuh, and report the faster one as e2e)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed command() (action, U, cost_total; theta for KMPPI) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "engine":
+        ap.error("--dump-outputs writes the engine's outputs (--impl engine)")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
-        run_reference(args, wl)      # bounds its own step count
+        run_reference(args, wl)
     else:
         run_engine(args, wl)
 

@@ -6,6 +6,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -38,6 +40,29 @@ def test_engine_arm_refuses_to_run_without_a_gpu():
                        capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert r.returncode != 0
     assert not any(ln.startswith('{"metric"') for ln in r.stdout.splitlines())
+
+
+@pytest.mark.gpu
+def test_engine_arm_dumps_the_last_timed_command(tmp_path):
+    """`--dump-outputs`: what the last timed command() returned to its caller, as .npy files that two runs with the same
+    arguments reproduce; `--steps` sets the length of every timed loop."""
+    import numpy as np
+    outs = []
+    for run in range(2):
+        d = tmp_path / f"run{run}"
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "nav2d_c3", "--steps", "7",
+                            "--warmup", "2", "--no-cpu-baseline", "--dump-outputs", str(d)],
+                           capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert r.returncode == 0, r.stderr[-2000:]
+        line = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1])
+        assert line["steps"] == 7 and line["config"]["step_stats_ms"]["n"] == 7 and line["e2e"]["steps"] == 7
+        outs.append({p.stem: np.load(p) for p in d.glob("*.npy")})
+    a = outs[0]
+    assert sorted(a) == ["U", "action", "cost_total", "theta"]
+    assert a["action"].shape == (2,) and a["U"].shape == (40, 2) and a["cost_total"].shape == (8192,) and a["theta"].shape == (5, 2)
+    assert all(v.dtype == np.float32 and np.isfinite(v).all() for v in a.values())
+    for k in a:
+        np.testing.assert_array_equal(a[k], outs[1][k], err_msg=k)
 
 
 def test_bench_helpers_statistics_bytes_and_workloads():
