@@ -547,7 +547,8 @@ __device__ void fold_tile(const KArgs<real>& a, Smem<real>& sm, real c_tot, bool
     // only the rollout threads (tid < BS) carry a cost; the helper threads contribute +inf / 0
     const real tile_min = block_min<real>(c_tot, sm.red);
     const real beta_new = tile_min < beta_run ? tile_min : beta_run;
-    const real w = active ? O::exp_(nfl * (c_tot - beta_new)) : (real)0;                  // mppi.py:12-13, 256
+    // no finite cost yet (every sample so far infeasible): weight 0, not exp(inf - inf) = NaN
+    const real w = (active && beta_new != O::inf()) ? O::exp_(nfl * (c_tot - beta_new)) : (real)0;   // mppi.py:12-13, 256
     const real resc = (beta_run == O::inf()) ? (real)0 : O::exp_(nfl * (beta_run - beta_new));
     if (tid < BS) sm.w_s[tid] = w;
     w_out = w;
@@ -1035,9 +1036,13 @@ __device__ __noinline__ void combine_records(const double* recs, int nrec, int R
     __syncthreads();
     double beta = part2[0];
     for (int w = 1; w < nw; ++w) beta = fmin(beta, part2[w]);
-    // the rescale factors in the controller's precision (exact for equal betas; beta_q - beta is exact in fp64)
-    if (tid < nrec) sq[tid] = (double)O::exp_((real)(nfl * (b_mine - beta)));
-    for (int q = tid + BD; q < nrec; q += BD) sq[q] = (double)O::exp_((real)(nfl * (recs[(size_t)q * RW] - beta)));
+    // the rescale factors in the controller's precision (exact for equal betas; beta_q - beta is exact in fp64); an empty
+    // record weighs 0
+    if (tid < nrec) sq[tid] = b_mine == (double)INFINITY ? 0.0 : (double)O::exp_((real)(nfl * (b_mine - beta)));
+    for (int q = tid + BD; q < nrec; q += BD) {
+        const double bq = recs[(size_t)q * RW];
+        sq[q] = bq == (double)INFINITY ? 0.0 : (double)O::exp_((real)(nfl * (bq - beta)));
+    }
     __syncthreads();
     if (tid == 0) numd[0] = beta;
     // the loads of a batch are issued together, THEN used: written as `acc += sq[q] * recs[..]` in one loop, ptxas keeps
