@@ -244,9 +244,9 @@ template <typename real, int V, int NU>
 int run_softmin(const MppiFusedParams* p, const void* cost, const void* eps, cudaStream_t stream) {
     auto kernel = softmin_update_kernel<real, V, NU>;
     Geometry g;
-    int rc = plan_geometry(kernel, p, (int)sizeof(real), 0, false, g, layout_fn<real>);
+    int rc = plan_geometry(kernel, p, (int)sizeof(real), ticket_layout_extra(p), false, g, layout_fn<real>);
     if (rc) return rc;
-    const uint64_t need_ws = ws_bytes(g.nb, rows_of(p), (int)sizeof(real));
+    const uint64_t need_ws = ws_bytes(g.nb, rows_of(p));
     if (p->workspace == nullptr || p->workspace_bytes < need_ws) return MPPI_ERR_WORKSPACE;
     if (p->n_env > 1 && (p->env_ws_stride < need_ws || p->workspace_bytes < p->env_ws_stride * (uint64_t)p->n_env)) return MPPI_ERR_WORKSPACE;
     KArgs<real> a;
@@ -540,10 +540,10 @@ int mppi_apply_partials(const MppiFusedParams* p, const void* partials, void* st
     return MPPI_ERR_BAD_ARG;
 }
 
-// two epoch parities of MPPI_XCHG_PARITY_WORDS flagged 8-byte words: world x records x 2 (R+2) words per command (the
-// fused kernel's record layout), or the stepped route's [source rank][MPPI_XCHG_MAX_WORDS] layout — both fit
+// two epoch parities of MPPI_XCHG_PARITY_WORDS flagged 8-byte words, records of 2 (R+2) words: world x records per command
+// (LL mode: every rank's cluster records, at most the 48 KB staging; rank-record mode: one record per rank)
 uint64_t mppi_xchg_bytes(void) { return (uint64_t)2 * MPPI_XCHG_PARITY_WORDS * sizeof(unsigned long long); }
-static_assert(MPPI_MAX_RANKS * MPPI_XCHG_MAX_WORDS <= MPPI_XCHG_PARITY_WORDS, "mailbox parity too small for the rank-record layout");
+static_assert(MPPI_MAX_RANKS * MPPI_XCHG_MAX_WORDS <= MPPI_XCHG_PARITY_WORDS, "mailbox parity too small for one record per rank");
 
 int mppi_xchg_create(void** mailbox, void* ipc_handle_out_64B) {
     if (mailbox == nullptr || ipc_handle_out_64B == nullptr) return MPPI_ERR_BAD_ARG;

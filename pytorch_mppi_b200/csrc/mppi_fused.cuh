@@ -8,13 +8,13 @@
 //   B. colour with the Cholesky factor, add the nominal sequence (staged in shared memory by a TMA
 //      bulk copy), clamp -> the tile now holds the perturbed actions (KMPPI: the control points)
 //   C. T-step rollout with the state in registers, cost accumulated in the reference's op order
-//   D. online-softmin fold of the tile into the CTA's running partial (beta_b, eta_b, V_b[R])
-// The last CTA to finish (atomic ticket) rescales all CTA partials to the global beta, optionally
-// exchanges the rank partial with peer GPUs through NVLink mailboxes, and writes the updated nominal
-// sequence: `U += sum_k w_k eps_k / eta` lands without a second launch.
+//   D. online-softmin fold: every rollout warp folds its 32 samples into its own running record (warp_fold)
+// The tail (warp_tail) combines the warp records of a CTA or cluster, then those of the grid (last arrival of an atomic
+// ticket, or a poller of flagged records), optionally exchanges the rank record with peer GPUs through NVLink mailboxes,
+// and writes the updated nominal sequence: `U += sum_k w_k eps_k / eta` lands without a second launch.
 //
 // sample_kernel / softmin_update_kernel: the same stages split at the Python T-loop, for arbitrary
-// dynamics/cost callables (A+B with coalesced write-out; D + finish from materialised tensors).
+// dynamics/cost callables (A+B with coalesced write-out; D + the same tail from materialised tensors).
 //
 // Reference lines replaced: mppi.py:232-238, 375-385, 297-332, 407-417, 254-259, 268-270
 // (SMPPI :489-493, 520-570; KMPPI :617-619, 657-688).
@@ -62,10 +62,7 @@ template <typename real> struct KArgs {
     real* z_out;
     // workspace carve
     unsigned int* ticket;
-    real* betaP;
-    real* etaP;
-    real* VP;
-    double* crec;                 // cluster records (n_clusters, R+2) doubles: (beta, eta, V[R]) — overlays betaP/etaP/VP
+    double* crec;                 // cluster records (n_clusters, R+2) doubles: (beta, eta, V[R])
     // multi-GPU
     unsigned long long* peers[8];
     double* partial_out;
@@ -107,8 +104,8 @@ template <typename real> struct KArgs {
 
 // ---- shared-memory carve, computed identically on host and device -------------------------------
 struct SmemLayout {
-    int off_uraw, off_araw, off_thraw, off_us, off_as, off_ths, off_w, off_wsh, off_vrun, off_ws, off_red,
-        off_part, off_rows, off_rows2, off_ss, off_part2, off_numd, off_redd, off_xs, off_wrec, off_xstage, off_sqd, total;
+    int off_uraw, off_araw, off_thraw, off_us, off_as, off_ths, off_w, off_wsh, off_rows, off_rows2, off_part2, off_numd,
+        off_xs, off_wrec, off_xstage, off_sqd, total;
     int LD;
 };
 
@@ -121,10 +118,11 @@ __host__ __device__ inline int layout_extra(int rows2, int nx_split, int cluster
 
 __host__ __device__ inline int align_up(int x, int a) { return (x + a - 1) / a * a; }
 
-// rows2 (a second TN-row tile) is only used by sample_kernel for KMPPI
 // BD = threads per CTA, BS = samples per tile (BD / threads-per-sample)
-// `extra`: bit 0 = rows2 needed; bits 8.. = nx of the split-cost rollout's per-step state buffer xs[T*nx][BS]
-// (0 = none; see fused_command_kernel<..., SPLIT>)
+// `extra` (layout_extra): bit 0 = rows2 tile (a second TN-row tile: the fused kernels' SMPPI / KMPPI tile, sample_kernel's
+// KMPPI trajectories); bits 8.. = nx of the split-cost rollout's per-step state buffer xs[T*nx][BS] (0 = none; see
+// fused_command_kernel<..., SPLIT>); the warp-record area and the finisher's staging (see above)
+// nb = records the finisher reads from the L2 workspace (ticket mode; 1 otherwise): their rescale factors live in sqd
 template <typename real>
 __host__ __device__ inline SmemLayout make_layout(int variant, int T, int nu, int S, int R, int BD, int BS, int nb, int extra) {
     SmemLayout L;
@@ -140,17 +138,12 @@ __host__ __device__ inline SmemLayout make_layout(int variant, int T, int nu, in
     L.off_ths = o; o = align_up(o + (variant == V_KMPPI ? SN : 0) * es, 16);
     L.off_w = o; o = align_up(o + (variant == V_KMPPI ? T * S : 0) * es, 16);
     L.off_wsh = o; o = align_up(o + (variant == V_KMPPI ? S * S : 0) * es, 16);
-    L.off_vrun = o; o = align_up(o + R * es, 16);
-    L.off_ws = o; o = align_up(o + BS * es, 16);
-    L.off_red = o; o = align_up(o + 64 * es, 16);
-    L.off_part = o; o = align_up(o + nw * R * es, 16);
     L.LD = BS + 1;
     L.off_rows = o; o = align_up(o + R * L.LD * es, 16);
     L.off_rows2 = o; o = align_up(o + (need_rows2 ? TN * L.LD : 0) * es, 16);
-    L.off_ss = o; o = align_up(o + 2 * nb * es, 16);
-    L.off_part2 = o; o = align_up(o + nw * R * 8, 16);
+    // combine_*: (BD / 64) groups x (R + 1) columns, and one group in a CTA of one warp
+    L.off_part2 = o; o = align_up(o + (nw > 1 ? nw * R : R + 1) * 8, 16);
     L.off_numd = o; o = align_up(o + (R + 2) * 8, 16);
-    L.off_redd = o; o = align_up(o + 64 * 8, 16);
     L.off_xs = o; o = align_up(o + T * nx_split * BS * es, 16);
     // warp-fold tail: (cluster x rollout warps) records of (R+2) doubles — slots [0, BS/32) are this CTA's own running
     // records, the cluster leader also receives its peers' through distributed shared memory
@@ -168,8 +161,8 @@ __host__ __device__ inline SmemLayout make_layout(int variant, int T, int nu, in
     return L;
 }
 
-#define MPPI_XCHG_MAX_R 1024
-#define MPPI_XCHG_MAX_WORDS (2 * (MPPI_XCHG_MAX_R + 2))
+#define MPPI_XCHG_MAX_R 1024                            // rows of a record a sharded controller exchanges
+#define MPPI_XCHG_MAX_WORDS (2 * (MPPI_XCHG_MAX_R + 2))  // mailbox words of such a record
 
 #if defined(__CUDACC__)
 
@@ -210,7 +203,7 @@ __device__ __forceinline__ void stamp(unsigned long long* dbg, int slot) {
     }
 }
 
-// ---- block reductions (deterministic: fixed shuffle tree, fixed warp order) ----------------------
+// ---- warp reductions (deterministic: fixed shuffle tree) -----------------------------------------
 template <typename T> __device__ __forceinline__ T warp_min(T v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
@@ -224,33 +217,12 @@ template <typename T> __device__ __forceinline__ T warp_sum(T v) {
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
 }
-// all threads get the result; `red` has >= 32 entries; each contains two __syncthreads
-template <typename T> __device__ __forceinline__ T block_min(T v, T* red) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
-    v = warp_min(v);
-    __syncthreads();
-    if (lane == 0) red[warp] = v;
-    __syncthreads();
-    T r = red[0];
-    for (int i = 1; i < nw; ++i) r = red[i] < r ? red[i] : r;
-    return r;
-}
-template <typename T> __device__ __forceinline__ T block_sum(T v, T* red) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
-    v = warp_sum(v);
-    __syncthreads();
-    if (lane == 0) red[warp] = v;
-    __syncthreads();
-    T r = red[0];
-    for (int i = 1; i < nw; ++i) r += red[i];
-    return r;
-}
 
 // ---- shared-memory view ---------------------------------------------------------------------
 template <typename real> struct Smem {
     unsigned long long* bar;
-    real *Uraw, *Araw, *thraw, *Us, *As, *ths, *Ws, *Wsh, *Vrun, *w_s, *red, *part, *rows, *rows2, *sS, *xs;
-    double *part2, *numd, *redd, *wrec, *xstage, *sqd;
+    real *Uraw, *Araw, *thraw, *Us, *As, *ths, *Ws, *Wsh, *rows, *rows2, *xs;
+    double *part2, *numd, *wrec, *xstage, *sqd;
     int LD;
     __device__ Smem(unsigned char* smem, const SmemLayout& L) {
         bar = reinterpret_cast<unsigned long long*>(smem);
@@ -262,16 +234,10 @@ template <typename real> struct Smem {
         ths = reinterpret_cast<real*>(smem + L.off_ths);
         Ws = reinterpret_cast<real*>(smem + L.off_w);
         Wsh = reinterpret_cast<real*>(smem + L.off_wsh);
-        Vrun = reinterpret_cast<real*>(smem + L.off_vrun);
-        w_s = reinterpret_cast<real*>(smem + L.off_ws);
-        red = reinterpret_cast<real*>(smem + L.off_red);
-        part = reinterpret_cast<real*>(smem + L.off_part);
         rows = reinterpret_cast<real*>(smem + L.off_rows);
         rows2 = reinterpret_cast<real*>(smem + L.off_rows2);
-        sS = reinterpret_cast<real*>(smem + L.off_ss);
         part2 = reinterpret_cast<double*>(smem + L.off_part2);
         numd = reinterpret_cast<double*>(smem + L.off_numd);
-        redd = reinterpret_cast<double*>(smem + L.off_redd);
         xs = reinterpret_cast<real*>(smem + L.off_xs);
         wrec = reinterpret_cast<double*>(smem + L.off_wrec);
         xstage = reinterpret_cast<double*>(smem + L.off_xstage);
@@ -302,7 +268,6 @@ __device__ void stage_issue(const KArgs<real>& a, Smem<real>& sm) {
             if (VARIANT == V_SMPPI) sm.Araw[j] = a.A[j];
         }
     }
-    for (int j = tid; j < R; j += BD) sm.Vrun[j] = (real)0;
     if (VARIANT == V_KMPPI) {
         for (int j = tid; j < R; j += BD) sm.thraw[j] = a.theta[j];
         for (int j = tid; j < T * S; j += BD) sm.Ws[j] = a.W[j];
@@ -534,60 +499,8 @@ __device__ __forceinline__ real eps_of(const NoiseModel<real>& nm, real val, rea
     return O::sub(val, as_or_ths);                                                          // mppi.py:664
 }
 
-// ---- stage D: fold one tile into the CTA's running softmin partial --------------------------------
-// rows hold v / theta_k (EPS_DIRECT=false) or eps itself (EPS_DIRECT=true)
-template <typename real, int VARIANT, bool EPS_DIRECT>
-__device__ void fold_tile(const KArgs<real>& a, Smem<real>& sm, real c_tot, bool active, int nvalid, real& beta_run,
-                          real& eta_run, real& w_out) {
-    typedef Ops<real> O;
-    const int tid = threadIdx.x, BD = blockDim.x, lane = tid & 31, warp = tid >> 5;
-    const int BS = BD / a.tps, ng = BS >> 5;          // sample groups of 32 in the tile
-    const int R = a.R, LD = sm.LD;
-    const real nfl = a.nm.neg_inv_lambda;
-    // only the rollout threads (tid < BS) carry a cost; the helper threads contribute +inf / 0
-    const real tile_min = block_min<real>(c_tot, sm.red);
-    const real beta_new = tile_min < beta_run ? tile_min : beta_run;
-    // no finite cost yet (every sample so far infeasible): weight 0, not exp(inf - inf) = NaN
-    const real w = (active && beta_new != O::inf()) ? O::exp_(nfl * (c_tot - beta_new)) : (real)0;   // mppi.py:12-13, 256
-    const real resc = (beta_run == O::inf()) ? (real)0 : O::exp_(nfl * (beta_run - beta_new));
-    if (tid < BS) sm.w_s[tid] = w;
-    w_out = w;
-    __syncthreads();
-    // warp -> (sample group gi, row slice ri): every (gi, j) is produced by exactly one warp;
-    // the ri == 0 warps also reduce their group's 32 weights (the eta partial)
-    const int gi = warp % ng, ri = warp / ng;
-    if (ri == 0) {
-        const int i = gi * 32 + lane;
-        const real wsum = warp_sum<real>(i < nvalid ? sm.w_s[i] : (real)0);
-        if (lane == 0) sm.red[32 + gi] = wsum;
-    }
-    for (int j = lane + 32 * ri; j < R; j += 32 * a.tps) {
-        const real us = (VARIANT == V_KMPPI || EPS_DIRECT) ? (real)0 : sm.Us[j];
-        const real a2 = EPS_DIRECT ? (real)0 : (VARIANT == V_SMPPI ? sm.As[j] : (VARIANT == V_KMPPI ? sm.ths[j] : (real)0));
-        real acc = (real)0;
-        const int i0 = gi * 32;
-        const int i1 = min(i0 + 32, nvalid);
-        for (int i = i0; i < i1; ++i) {
-            const real val = sm.rows[j * LD + i];
-            acc += sm.w_s[i] * (EPS_DIRECT ? val : eps_of<real, VARIANT>(a.nm, val, us, a2));   // mppi.py:268
-        }
-        sm.part[gi * R + j] = acc;
-    }
-    __syncthreads();
-    for (int j = tid; j < R; j += BD) {
-        real s = sm.part[j];
-        for (int q = 1; q < ng; ++q) s += sm.part[q * R + j];
-        sm.Vrun[j] = sm.Vrun[j] * resc + s;
-    }
-    real eta_tile = sm.red[32];
-    for (int q = 1; q < ng; ++q) eta_tile += sm.red[32 + q];
-    eta_run = eta_run * resc + eta_tile;
-    beta_run = beta_new;
-    __syncthreads();
-}
-
-// ---- peer exchange over NVLink mailboxes (LL-style 8-byte records: payload32 | flag32) ----------
-// mailbox layout per rank: [2 parity][MPPI_MAX_RANKS src][MPPI_XCHG_MAX_WORDS] u64
+// ---- flagged 8-byte words (payload32 | flag32): peer mailboxes, the local record mailbox, host delivery ----------
+// (the record layout of a mailbox: xchg_publish_words below)
 // relaxed.sys, not volatile: the words are self-validating, so nothing orders one against another — and ptxas completes
 // every volatile access before it issues the next (a thread polling 8 words paid 8 L2 round trips per sweep; the same
 // serialisation made a 32-record combine from shared memory cost 1.5 us)
@@ -598,53 +511,6 @@ __device__ __forceinline__ unsigned long long ld_poll(const unsigned long long* 
     unsigned long long v;
     asm volatile("ld.relaxed.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
     return v;
-}
-
-// numd[0]=beta, numd[1]=eta, numd[2..2+R) = numerators of THIS rank; on return they hold the
-// all-rank combination (bit-identical on every rank).  Returns 0, or 1 on timeout.
-template <typename real>
-__device__ int exchange_partials(const KArgs<real>& a, double* numd, double* scratch /*world*(R+2)*/, double nfl) {
-    const int R = a.R, nwords = 2 * (R + 2);
-    const int tid = threadIdx.x, BD = blockDim.x;
-    const uint32_t flag = (uint32_t)(a.epoch & 0x7fffffffull) | 0x80000000u;
-    const size_t par_off = (size_t)(a.epoch & 1ull) * 8 * MPPI_XCHG_MAX_WORDS;
-    __shared__ int s_timeout;
-    if (tid == 0) s_timeout = 0;
-    __syncthreads();
-    for (int i = tid; i < nwords; i += BD) {
-        unsigned long long bits = (unsigned long long)__double_as_longlong(numd[i >> 1]);
-        uint32_t half = (i & 1) ? (uint32_t)(bits >> 32) : (uint32_t)bits;
-        unsigned long long rec = ((unsigned long long)flag << 32) | half;
-        for (int g = 0; g < a.world; ++g) st_peer(a.peers[g] + par_off + (size_t)a.rank * MPPI_XCHG_MAX_WORDS + i, rec);
-    }
-    const unsigned long long* mine = a.peers[a.rank] + par_off;
-    const long long t0 = clock64();
-    for (int e = tid; e < a.world * nwords; e += BD) {
-        const int g = e / nwords, i = e - g * nwords;
-        unsigned long long rec;
-        while (true) {
-            rec = ld_poll(mine + (size_t)g * MPPI_XCHG_MAX_WORDS + i);
-            if ((uint32_t)(rec >> 32) == flag) break;
-            if (clock64() - t0 > 4000000000ll) { s_timeout = 1; break; }
-        }
-        reinterpret_cast<uint32_t*>(scratch)[(size_t)g * nwords + i] = (uint32_t)rec;
-    }
-    __syncthreads();
-    if (s_timeout) return 1;
-    double beta = scratch[0];
-    for (int g = 1; g < a.world; ++g) beta = fmin(beta, scratch[(size_t)g * (R + 2)]);
-    __syncthreads();
-    for (int j = tid; j < R + 1; j += BD) {   // j==0 -> eta, j>=1 -> numerator j-1
-        double acc = 0.0;
-        for (int g = 0; g < a.world; ++g) {
-            const double* rec = scratch + (size_t)g * (R + 2);
-            acc += exp(nfl * (rec[0] - beta)) * rec[1 + j];
-        }
-        numd[1 + j] = acc;
-    }
-    if (tid == 0) numd[0] = beta;
-    __syncthreads();
-    return 0;
 }
 
 // value i of the action as flagged 8-byte word(s) in pinned host memory (float: 1 word, double: 2)
@@ -727,198 +593,10 @@ __device__ void finish_update(const KArgs<real>& a, const double* numd, const re
     }
 }
 
-// ---- tail: publish the CTA partial; the last CTA combines, exchanges, updates ----------------------
-// Returns true in the CTA that finished the command (the last arrival), false in all the others.
-template <typename real, int VARIANT, int NU>
-__device__ bool publish_and_finish(const KArgs<real>& a, Smem<real>& sm, real beta_run, real eta_run) {
-    typedef Ops<real> O;
-    const int tid = threadIdx.x, BD = blockDim.x, lane = tid & 31, warp = tid >> 5, nw = BD >> 5;
-    const int R = a.R, TN = a.TN;
-    const real nfl = a.nm.neg_inv_lambda;
-    __shared__ int s_is_last;
-    const int b = blockIdx.x;
-    if (tid == 0) {
-        a.betaP[b] = beta_run;
-        a.etaP[b] = eta_run;
-    }
-    for (int j = tid; j < R; j += BD) a.VP[(size_t)b * R + j] = sm.Vrun[j];
-    // release: the CTA barrier orders every thread's stores before thread 0, whose single gpu-scope
-    // fence + ticket increment publishes them (one MEMBAR per CTA instead of one per warp)
-    __syncthreads();
-    if (tid == 0) {
-        // one acq_rel ticket increment: releases this CTA's record (the barrier above made every thread's
-        // stores visible to thread 0) and, for the last arrival, acquires all the others' — cheaper than
-        // the two sequentially-consistent fences __threadfence() would insert around a relaxed atomic
-        unsigned int t;
-        asm volatile("atom.acq_rel.gpu.global.add.u32 %0, [%1], %2;" : "=r"(t) : "l"(a.ticket), "r"(1u) : "memory");
-        s_is_last = (t == gridDim.x - 1);
-    }
-    __syncthreads();
-    stamp(a.dbg, 6);
-    if (!s_is_last) return false;
-    stamp(a.dbg, 8);
-
-    // The partials were written by other SMs before their ticket increments; this CTA has not
-    // touched those lines during this launch, and __ldcg reads them from L2.  Every load whose
-    // address does not depend on beta is issued up front (one L2 round trip for the common case);
-    // the scalar part (beta, rescale factors, eta) is spread over all threads.
-    const int nb = gridDim.x;
-    const real* betaP = a.betaP;
-    const real* etaP = a.etaP;
-    const real* VP = a.VP;
-    real* sB = sm.sS;            // [nb] beta_q, then rescale factors s_q
-    real* sE = sm.sS + nb;       // [nb] eta_q
-    // 1) issue every load whose address is known now: this thread's scalars and the first 16 records of
-    //    its (warp, lane) numerator slice — one L2 round trip covers the common case completely
-    constexpr int PF = 16;
-    real vpre[PF];
-#pragma unroll
-    for (int u = 0; u < PF; ++u) {
-        const int q = warp + u * nw;
-        vpre[u] = (lane < R && q < nb) ? __ldcg(VP + (size_t)q * R + lane) : (real)0;
-    }
-    if (nb <= 256) {
-        // small grids: warp 0 alone, shuffles only, ONE barrier (measured faster than block-wide
-        // reductions here: 16 warps' barriers cost more than 8 loads per lane)
-        if (warp == 0) {
-            real b8[8], e8[8];
-#pragma unroll
-            for (int u = 0; u < 8; ++u) {
-                const int q = lane + 32 * u;
-                b8[u] = q < nb ? __ldcg(betaP + q) : O::inf();
-                e8[u] = q < nb ? __ldcg(etaP + q) : (real)0;
-            }
-            real bl = b8[0];
-#pragma unroll
-            for (int u = 1; u < 8; ++u) bl = b8[u] < bl ? b8[u] : bl;
-            const real beta = warp_min<real>(bl);
-            double el = 0.0;
-#pragma unroll
-            for (int u = 0; u < 8; ++u) {
-                const int q = lane + 32 * u;
-                if (q < nb) {
-                    const real sq = O::exp_(nfl * (b8[u] - beta));
-                    sB[q] = sq;
-                    el += (double)sq * (double)e8[u];
-                }
-            }
-            const double eta = warp_sum<double>(el);
-            if (lane == 0) {
-                sm.numd[0] = (double)beta;
-                sm.numd[1] = eta;
-                *a.ticket = 0u;   // self-reset: the next launch needs no memset
-            }
-        }
-        __syncthreads();
-    } else {
-        real bq0 = O::inf(), eq0 = (real)0, bq1 = O::inf(), eq1 = (real)0;
-        if (tid < nb) {
-            bq0 = __ldcg(betaP + tid);
-            eq0 = __ldcg(etaP + tid);
-        }
-        if (tid + BD < nb) {
-            bq1 = __ldcg(betaP + tid + BD);
-            eq1 = __ldcg(etaP + tid + BD);
-        }
-        real bl = bq0 < bq1 ? bq0 : bq1;
-        for (int q = tid + 2 * BD; q < nb; q += BD) {          // very large grids only
-            const real bq = __ldcg(betaP + q);
-            sB[q] = bq;
-            sE[q] = __ldcg(etaP + q);
-            bl = bq < bl ? bq : bl;
-        }
-        const real beta = block_min<real>(bl, sm.red);
-        double el = 0.0;
-        if (tid < nb) {
-            const real sq = O::exp_(nfl * (bq0 - beta));
-            sB[tid] = sq;
-            el += (double)sq * (double)eq0;
-        }
-        if (tid + BD < nb) {
-            const real sq = O::exp_(nfl * (bq1 - beta));
-            sB[tid + BD] = sq;
-            el += (double)sq * (double)eq1;
-        }
-        for (int q = tid + 2 * BD; q < nb; q += BD) {
-            const real sq = O::exp_(nfl * (sB[q] - beta));
-            sB[q] = sq;
-            el += (double)sq * (double)sE[q];
-        }
-        const double eta = block_sum<double>(el, sm.redd);   // its barriers also publish sB
-        if (tid == 0) {
-            sm.numd[0] = (double)beta;
-            sm.numd[1] = eta;
-            *a.ticket = 0u;   // self-reset: the next launch needs no memset
-        }
-    }
-    stamp(a.dbg, 10);
-    // 3) numerators: rows j = lane (+32..), records q = warp (+nw..), PF loads in flight per thread
-    for (int j = lane; j < R; j += 32) {
-        double acc = 0.0;
-        int q = warp;
-        if (j == lane) {
-#pragma unroll
-            for (int u = 0; u < PF; ++u) {
-                const int qq = warp + u * nw;
-                if (qq < nb) acc += (double)sB[qq] * (double)vpre[u];
-            }
-            q = warp + PF * nw;
-        }
-        for (; q < nb; q += PF * nw) {
-            real v[PF];
-#pragma unroll
-            for (int u = 0; u < PF; ++u) {
-                const int qq = q + u * nw;
-                v[u] = qq < nb ? __ldcg(VP + (size_t)qq * R + j) : (real)0;
-            }
-#pragma unroll
-            for (int u = 0; u < PF; ++u) {
-                const int qq = q + u * nw;
-                if (qq < nb) acc += (double)sB[qq] * (double)v[u];
-            }
-        }
-        sm.part2[warp * R + j] = acc;
-    }
-    __syncthreads();
-    for (int j = tid; j < R; j += BD) {
-        double s2 = sm.part2[j];
-        for (int q = 1; q < nw; ++q) s2 += sm.part2[q * R + j];
-        sm.numd[2 + j] = s2;
-    }
-    __syncthreads();
-    stamp(a.dbg, 11);
-
-    if (a.export_partial) {   // library-collective route: caller all-gathers, mppi_apply_partials finishes
-        for (int j = tid; j < R + 2; j += BD) a.partial_out[j] = sm.numd[j];
-        for (int j = tid; j < TN; j += BD) {
-            a.nominal_used[j] = sm.Us[j];
-            if (VARIANT == V_SMPPI) a.nominal_used[TN + j] = sm.As[j];
-        }
-        if (VARIANT == V_KMPPI)
-            for (int j = tid; j < R; j += BD) a.nominal_used[2 * TN + j] = sm.ths[j];
-        if (tid == 0) {
-            a.stats[0] = sm.numd[0];
-            a.stats[1] = sm.numd[1];
-            a.stats[3] = 0.0;
-        }
-        return true;
-    }
-    if (a.world > 1) {
-        double* scratch = reinterpret_cast<double*>(sm.rows);   // the tile is free now
-        if (exchange_partials<real>(a, sm.numd, scratch, (double)nfl)) {
-            if (tid == 0) a.stats[3] = -6.0;   // MPPI_ERR_TIMEOUT
-            return true;
-        }
-    }
-    finish_update<real, VARIANT>(a, sm.numd, sm.Us, sm.As, sm.ths, sm.Ws, NU);
-    if (tid == 0) a.stats[3] = 0.0;
-    return true;
-}
-
-
 // =================================================================================================
-// Warp-fold tail (fused_command_kernel): the softmin reduction without CTA-wide barriers in the fold, a
-// thread-block-cluster stage through distributed shared memory, and a finisher that works on a handful of records.
+// Warp-fold tail: the softmin reduction of every command kernel (fused, resident, tcgen05 and the stepped route's
+// softmin_update_kernel) — no CTA-wide barriers in the fold, a thread-block-cluster stage through distributed shared
+// memory (fused / resident kernels), and a finisher that works on a handful of records.
 //
 //   per tile   each ROLLOUT WARP folds its 32 samples into its own running record (beta_w, eta_w, V_w[R]) — shuffles
 //              only, fp64 accumulation, record in shared memory (warp-private: no barrier)
@@ -968,15 +646,21 @@ __device__ __forceinline__ void warp_records_init(const KArgs<real>& a, Smem<rea
 }
 
 // ---- per tile: fold this warp's 32 samples into its running record (rollout warps only; warp-synchronous) ----------
-template <typename real, int VARIANT>
+// Where the weighted quantity of row j comes from:
+enum {
+    FOLD_ROWS = 0,    // eps_of(rows): the tile holds the perturbed actions / control points
+    FOLD_ROWS2 = 1,   // rows2 holds the effective noise (SMPPI with TILE2: written once by transform_column)
+    FOLD_EPS = 2      // rows holds eps itself (softmin_update_kernel: the materialised noise)
+};
+template <typename real, int VARIANT, int SRC>
 __device__ __forceinline__ void warp_fold(const KArgs<real>& a, Smem<real>& sm, real c_tot, bool active, int nvalid) {
     typedef Ops<real> O;
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     const int R = a.R, LD = sm.LD, i0 = w * 32;
     double* rec = sm.wrec + (size_t)w * (R + 2);
     const real nfl = a.nm.neg_inv_lambda;
-    // the 32 columns this warp reads below were written by its own lanes (one sample per thread: no CTA barrier in
-    // between) — order them
+    // the fused kernels: the 32 columns this warp reads below were written by its own lanes (one sample per thread: no
+    // CTA barrier in between) — order them.  (Kernels whose tile is written by other warps put a CTA barrier first.)
     __syncwarp();
     const real cmin = warp_min<real>(active ? c_tot : O::inf());
     const real beta_run = (real)rec[0];                 // a value of type `real`, kept in a double slot
@@ -990,17 +674,16 @@ __device__ __forceinline__ void warp_fold(const KArgs<real>& a, Smem<real>& sm, 
         const int j = jb + lane;
         const bool jv = j < R;
         const int jc = jv ? j : 0;
-        const real us = (VARIANT == V_KMPPI) ? (real)0 : sm.Us[jc];
-        const real a2 = VARIANT == V_SMPPI ? sm.As[jc] : (VARIANT == V_KMPPI ? sm.ths[jc] : (real)0);
-        // SMPPI: the tile of effective noise (rows2, written once by transform_column) — no division here
-        const real* row = (VARIANT == V_SMPPI ? sm.rows2 : sm.rows) + (size_t)jc * LD + i0;
+        const real us = (VARIANT == V_KMPPI || SRC != FOLD_ROWS) ? (real)0 : sm.Us[jc];
+        const real a2 = SRC != FOLD_ROWS ? (real)0 : (VARIANT == V_SMPPI ? sm.As[jc] : (VARIANT == V_KMPPI ? sm.ths[jc] : (real)0));
+        const real* row = (SRC == FOLD_ROWS2 ? sm.rows2 : sm.rows) + (size_t)jc * LD + i0;
         // the 32 products of a warp are added in the controller's precision (as the reference's einsum does, in its own
         // order); everything ACROSS warps, CTAs and GPUs is fp64 (measured: an fp64 inner sum costs the large-K
         // geometry, where every warp folds, 5 us per command through F2F.F64 / DADD issue)
         real acc = (real)0;
         for (int i = 0; i < nv; ++i) {
             const real wi = __shfl_sync(0xffffffffu, wgt, i);
-            const real e = VARIANT == V_SMPPI ? row[i] : eps_of<real, VARIANT>(a.nm, row[i], us, a2);
+            const real e = SRC == FOLD_ROWS ? eps_of<real, VARIANT>(a.nm, row[i], us, a2) : row[i];
             acc += wi * e;                                                                      // mppi.py:268
         }
         if (jv) rec[2 + j] = rec[2 + j] * resc + (double)acc;
@@ -1016,8 +699,8 @@ __device__ __forceinline__ void warp_fold(const KArgs<real>& a, Smem<real>& sm, 
 // ---- fixed-order fp64 combination of records (beta_q, eta_q, V_q[R]) -----------------------------------------------
 //   beta = min beta_q ; s_q = exp(nfl (beta_q - beta)) ; eta = sum s_q eta_q ; V[j] = sum s_q V_q[j]   -> numd[0 .. R+2)
 // CTA-wide (every thread calls it; three barriers).  Record q is recs[q * (R+2) ..] in shared or global memory (generic
-// pointer, volatile loads: L2 for global).  Threads are (group g = tid / 64, column jl = tid % 64): group g adds the
-// records q = g, g + nG, ... for its columns (column 0 = eta, column 1 + j = V[j]) into part2[g][..], the groups are added
+// pointer, volatile loads: L2 for global).  Threads are (group g = tid / W, column jl = tid % W; W = 64, or 32 in a CTA of
+// one warp, so that every group is complete): group g adds the records q = g, g + nG, ... for its columns (column 0 = eta, column 1 + j = V[j]) into part2[g][..], the groups are added
 // in order — the result does not depend on timing.  Deliberately SMALL and out of line (one copy for every call site):
 // the tail runs once per command on a cold instruction cache, where instruction count, not arithmetic, sets its time
 // (ncu: `no_instruction` is the third-largest stall of the kernel).
@@ -1026,7 +709,8 @@ __device__ __noinline__ void combine_records(const double* recs, int nrec, int R
                                              double* numd) {
     typedef Ops<real> O;
     const int RW = R + 2, C = R + 1;                      // columns: eta, V[0..R)
-    const int tid = threadIdx.x, BD = blockDim.x, nG = BD >> 6, g = tid >> 6, jl = tid & 63, nw = BD >> 5;
+    const int BD = blockDim.x, lw = BD < 64 ? 5 : 6, W = 1 << lw;
+    const int tid = threadIdx.x, nG = BD >> lw, g = tid >> lw, jl = tid & (W - 1), nw = BD >> 5;
     // beta: ONE load per thread (record tid; more only for grids above blockDim records), warp minima through sq[]
     const double b_mine = tid < nrec ? recs[(size_t)tid * RW] : (double)INFINITY;
     double b = b_mine;
@@ -1049,7 +733,7 @@ __device__ __noinline__ void combine_records(const double* recs, int nrec, int R
     // every volatile load next to its DFMA and a thread waits one L2 round trip per record (K = 131072: 293 records in
     // the L2 workspace, 42 per thread — 9 us; batched: 6 round trips)
     constexpr int UB = 8;
-    for (int j = jl; j < C; j += 64) {
+    for (int j = jl; j < C; j += W) {
         double acc = 0.0;
         const double* col = recs + 1 + j;
         for (int q0 = g; q0 < nrec; q0 += nG * UB) {
@@ -1084,7 +768,8 @@ template <typename real>
 __device__ __noinline__ void combine_global(const double* recs, int nrec, int R, double nfl, double* part2, double* sq, double* numd) {
     typedef Ops<real> O;
     const int RW = R + 2, C = R + 1;
-    const int tid = threadIdx.x, BD = blockDim.x, nG = BD >> 6, g = tid >> 6, jl = tid & 63, nw = BD >> 5;
+    const int BD = blockDim.x, lw = BD < 64 ? 5 : 6, W = 1 << lw;     // column groups of 64 (32 in a CTA of one warp)
+    const int tid = threadIdx.x, nG = BD >> lw, g = tid >> lw, jl = tid & (W - 1), nw = BD >> 5;
     double b = (double)INFINITY;
     for (int q = tid; q < nrec; q += BD) b = fmin(b, __ldcg(recs + (size_t)q * RW));
     b = warp_min<double>(b);
@@ -1099,7 +784,7 @@ __device__ __noinline__ void combine_global(const double* recs, int nrec, int R,
     __syncthreads();
     if (tid == 0) numd[0] = beta;
     constexpr int UB = 8;
-    for (int j = jl; j < C; j += 64) {
+    for (int j = jl; j < C; j += W) {
         double acc = 0.0;
         const double* col = recs + 1 + j;
         for (int q0 = g; q0 < nrec; q0 += nG * UB) {
@@ -1393,9 +1078,6 @@ __device__ void make_env_args(const KArgs<real>& in, KArgs<real>* out) {
         if (in.ticket) {
             const long long off = e * in.env_ws_stride;
             out->ticket = reinterpret_cast<unsigned int*>(reinterpret_cast<unsigned char*>(in.ticket) + off);
-            out->betaP = reinterpret_cast<real*>(reinterpret_cast<unsigned char*>(in.betaP) + off);
-            out->etaP = reinterpret_cast<real*>(reinterpret_cast<unsigned char*>(in.etaP) + off);
-            out->VP = reinterpret_cast<real*>(reinterpret_cast<unsigned char*>(in.VP) + off);
             out->crec = reinterpret_cast<double*>(reinterpret_cast<unsigned char*>(in.crec) + off);
             if (in.world == 1 || in.export_partial)      // this GPU's own record mailbox lives in the environment's workspace
                 out->peers[0] = reinterpret_cast<unsigned long long*>(reinterpret_cast<unsigned char*>(in.peers[0]) + off);
@@ -1630,7 +1312,7 @@ MPPI_UNROLL_N(MPPI_ROLLOUT_UNROLL)
         }
         if (tile == blockIdx.x) stamp(a.dbg, 4);
         // D. every rollout warp folds its 32 samples into its own running record (no CTA barrier)
-        if (tid < BS) warp_fold<real, VARIANT>(a, sm, c_tot, active, nvalid);
+        if (tid < BS) warp_fold<real, VARIANT, VARIANT == V_SMPPI ? FOLD_ROWS2 : FOLD_ROWS>(a, sm, c_tot, active, nvalid);
         if (tile == blockIdx.x) stamp(a.dbg, 5);
         if (tile + (int)gridDim.x < a.n_tiles) __syncthreads();      // the tile is refilled by the next pass
     }
@@ -1767,10 +1449,14 @@ __global__ void states_kernel(const real* __restrict__ pa, real* __restrict__ st
 
 // =================================================================================================
 // Generic path, part 2: softmin + weighted update from materialised cost_total (K) and eps (K,R)
-// (mppi.py:254-259, 268-270).  HBM-bound: reads 4*K*(R+1) bytes once, coalesced.
+// (mppi.py:254-259, 268-270).  HBM-bound: reads 4*K*(R+1) bytes once, coalesced.  The rollout warps fold the tile with
+// warp_fold, and the command finishes in warp_tail without a cluster: the grid's CTA records combine through the ticket
+// (one record per rank, exchanged with the peers, on a sharded controller).  Never LL mode: the launch may be captured
+// into a CUDA graph, whose replays would repeat an LL record's per-command tag.
+// (512, 1): without the minimum ptxas squeezes some instantiations to 64 registers and spills in the tail.
 // =================================================================================================
 template <typename real, int VARIANT, int NU>
-__global__ void __launch_bounds__(512) softmin_update_kernel(const __grid_constant__ KArgs<real> a_in) {
+__global__ void __launch_bounds__(512, 1) softmin_update_kernel(const __grid_constant__ KArgs<real> a_in) {
     typedef Ops<real> O;
     extern __shared__ __align__(16) unsigned char smem[];
     const int tid = threadIdx.x, BD = blockDim.x;
@@ -1778,9 +1464,11 @@ __global__ void __launch_bounds__(512) softmin_update_kernel(const __grid_consta
     if (a_in.n_env > 1) make_env_args<real, 0, NU>(a_in, reinterpret_cast<KArgs<real>*>(a_env_raw));
     const KArgs<real>& a = a_in.n_env > 1 ? *reinterpret_cast<const KArgs<real>*>(a_env_raw) : a_in;
     const int BS = BD / a.tps;
-    const SmemLayout L = make_layout<real>(VARIANT, a.T, NU, a.S, a.R, BD, BS, gridDim.x, 0);
+    const SmemLayout L = make_layout<real>(VARIANT, a.T, NU, a.S, a.R, BD, BS, fused_layout_nb((int)gridDim.x, 1),
+                                           layout_extra(0, 0, 1, fused_xstage_doubles(a.world > 1 && !a.export_partial, a.world, 1, a.R)));
     Smem<real> sm(smem, L);
     const int R = a.R, TN = a.TN, LD = sm.LD;
+    warp_records_init<real>(a, sm);
     // post-shift nominal comes from nominal_used (written by sample_kernel)
     for (int j = tid; j < TN; j += BD) {
         sm.Us[j] = a.nominal_used[j];
@@ -1790,9 +1478,6 @@ __global__ void __launch_bounds__(512) softmin_update_kernel(const __grid_consta
         for (int j = tid; j < R; j += BD) sm.ths[j] = a.nominal_used[2 * TN + j];
         for (int j = tid; j < a.T * a.S; j += BD) sm.Ws[j] = a.W[j];
     }
-    for (int j = tid; j < R; j += BD) sm.Vrun[j] = (real)0;
-    __syncthreads();
-    real beta_run = O::inf(), eta_run = (real)0;
     for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x) {
         const int k = tile * BS + tid;
         const bool active = tid < BS && k < a.K;
@@ -1804,10 +1489,11 @@ __global__ void __launch_bounds__(512) softmin_update_kernel(const __grid_consta
             sm.rows[j * LD + s] = a.in_eps[base + e];
         }
         const real c = active ? a.in_cost[k] : O::inf();
-        real w;
-        fold_tile<real, VARIANT, true>(a, sm, c, active, nvalid, beta_run, eta_run, w);   // first barrier inside publishes rows
+        __syncthreads();                                              // the tile was loaded by every warp
+        if (tid < BS) warp_fold<real, VARIANT, FOLD_EPS>(a, sm, c, active, nvalid);
+        if (tile + (int)gridDim.x < a.n_tiles) __syncthreads();      // the tile is refilled by the next pass
     }
-    publish_and_finish<real, VARIANT, NU>(a, sm, beta_run, eta_run);
+    warp_tail<real, VARIANT, NU>(a, sm);
 }
 
 // omega_k = exp(-(c_k - beta)/lambda) / eta from the stats a command left behind (mppi.py:256-258)

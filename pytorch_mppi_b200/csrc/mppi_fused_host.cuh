@@ -62,15 +62,13 @@ int choose_fused(const ModelKernels* mk, const MppiFusedParams*& p, MppiFusedPar
     if (tc_route) p = &p_tc;
     const int R = rows_of(p), es = (int)sizeof(real);
     const int world = p->world <= 0 ? 1 : p->world;
-    bool any_peer = false;
-    for (int g = 0; g < MPPI_MAX_RANKS; ++g) any_peer = any_peer || p->peer_slots[g] != nullptr;
-    const bool sharded = world > 1 && any_peer && !(p->flags & MPPI_FLAG_EXPORT_PARTIAL);
+    const bool sharded = sharded_in_kernel(p);
     MppiFusedParams pg = *p;
     if (p->K_geom > p->K) pg.K = p->K_geom;
     Geometry g;
     int rc;
     if (tc_route) {
-        rc = plan_geometry(kernel, &pg, es, 0, false, g, layout_fn<real>);
+        rc = plan_geometry(kernel, &pg, es, ticket_layout_extra(p), false, g, layout_fn<real>);
         g_tc_kernel = 0;
         if (rc) return rc;
         c = FusedChoice{kernel, g, 0, 0, 1};
@@ -163,7 +161,7 @@ int run_fused(const ModelKernels* mk, const MppiFusedParams* p, cudaStream_t str
     int rc = choose_fused<real>(mk, p, p_tc, c);
     if (rc) return rc;
     const Geometry& g = c.g;
-    const uint64_t need_ws = ws_bytes(g.nb, rows_of(p), (int)sizeof(real));
+    const uint64_t need_ws = ws_bytes(g.nb, rows_of(p));
     KArgs<real> a;
     finish_kargs<real>(p, c, a);
     if (info != nullptr) {
@@ -177,7 +175,7 @@ int run_fused(const ModelKernels* mk, const MppiFusedParams* p, cudaStream_t str
         info->max_blocks_per_sm = g.occ;
         info->sm_count = di.sm_count;
         // report the worst case so one allocation serves any later geometry for these dimensions
-        info->workspace_bytes = ws_bytes(di.sm_count * 16, rows_of(p), (int)sizeof(real));
+        info->workspace_bytes = ws_bytes(di.sm_count * 16, rows_of(p));
         info->tma_staging = a.tma_ok;
         info->split_cost = c.split;
         info->wide_regs = c.wide;
@@ -218,7 +216,7 @@ template <typename real> int build_plan(const ModelKernels* mk, const MppiFusedP
     pl->g = c.g;
     if (p->U == nullptr || p->cost_total == nullptr || p->nominal_used == nullptr || p->stats == nullptr || p->workspace == nullptr)
         return MPPI_ERR_BAD_ARG;
-    if (p->workspace_bytes < ws_bytes(pl->g.nb, rows_of(p), (int)sizeof(real))) return MPPI_ERR_WORKSPACE;
+    if (p->workspace_bytes < ws_bytes(pl->g.nb, rows_of(p))) return MPPI_ERR_WORKSPACE;
     if (mk->param_bytes > (int)sizeof(pl->mparams)) return UNSUPPORTED("model parameter block too large");
     KArgs<real>* a = reinterpret_cast<KArgs<real>*>(pl->kargs);
     finish_kargs<real>(p, c, *a);

@@ -134,6 +134,19 @@ inline int validate(const MppiFusedParams* p, bool fused = false) {
 
 inline int rows_of(const MppiFusedParams* p) { return (p->variant == MPPI_VARIANT_KMPPI ? p->S : p->T) * p->nu; }
 
+// a sharded controller whose kernel exchanges the records with its peers over NVLink (not through a library collective)
+inline bool sharded_in_kernel(const MppiFusedParams* p) {
+    bool any_peer = false;
+    for (int g = 0; g < MPPI_MAX_RANKS; ++g) any_peer = any_peer || p->peer_slots[g] != nullptr;
+    return p->world > 1 && any_peer && !(p->flags & MPPI_FLAG_EXPORT_PARTIAL);
+}
+
+// make_layout's `extra` word of a kernel that finishes in warp_tail without a cluster, in ticket mode (xchg_npub = 1): the
+// softmin_update_kernel and the tcgen05 kernel
+inline int ticket_layout_extra(const MppiFusedParams* p) {
+    return layout_extra(0, 0, 1, fused_xstage_doubles(sharded_in_kernel(p), p->world, 1, rows_of(p)));
+}
+
 template <typename real> void fill_noise_model(const MppiFusedParams* p, NoiseModel<real>& nm) {
     for (int i = 0; i < MPPI_MAX_NU; ++i) {
         nm.mu[i] = (real)p->noise_mu[i];
@@ -155,17 +168,12 @@ template <typename real> void fill_noise_model(const MppiFusedParams* p, NoiseMo
     nm.abs_cost = (p->flags & MPPI_FLAG_ABS_COST) ? 1 : 0;
 }
 
-// ticket + per-CTA partials (beta_b, eta_b, V_b[R]) of type `real` (stepped-route / resident / tensor-core tails), or
-// ticket + per-cluster records of (R + 2) doubles (fused kernel's warp-fold tail): the larger of the two
+// ticket + the records of (R + 2) doubles the warp-fold tail combines in ticket mode (one per cluster of the grid)
 // ... followed by this GPU's own record mailbox (single-GPU LL mode): two epoch parities of MPPI_LL_LOCAL_WORDS flagged words
 #define MPPI_LL_STAGE_BYTES 49152                          // finisher staging budget: LL mode needs xw x clusters x (R+2) x 8 <= this
 #define MPPI_LL_LOCAL_WORDS (2 * MPPI_LL_STAGE_BYTES / 8)  // words per parity of the local mailbox (2 words per double)
-inline uint64_t ws_partials_bytes(int nb, int R, int es) {
-    const uint64_t per_cta = 16 + 2 * (uint64_t)align_up(nb * es, 16) + (uint64_t)align_up(nb * R * es, 16);
-    const uint64_t per_cluster = 16 + (uint64_t)nb * (uint64_t)(R + 2) * 8;
-    return ((per_cta > per_cluster ? per_cta : per_cluster) + 255) / 256 * 256;
-}
-inline uint64_t ws_bytes(int nb, int R, int es) { return ws_partials_bytes(nb, R, es) + 2ull * MPPI_LL_LOCAL_WORDS * 8; }
+inline uint64_t ws_partials_bytes(int nb, int R) { return (16 + (uint64_t)nb * (uint64_t)(R + 2) * 8 + 255) / 256 * 256; }
+inline uint64_t ws_bytes(int nb, int R) { return ws_partials_bytes(nb, R) + 2ull * MPPI_LL_LOCAL_WORDS * 8; }
 
 inline unsigned long long xchg_timeout_ns() {
     // how long a shard waits for its peers' records before giving up (rank skew: a GC pause, a JIT build, a lazy module
@@ -214,9 +222,6 @@ template <typename real> int fill_kargs(const MppiFusedParams* p, KArgs<real>& a
     if (p->workspace != nullptr) {
         unsigned char* w = (unsigned char*)p->workspace;
         a.ticket = (unsigned int*)w;
-        a.betaP = (real*)(w + 16);
-        a.etaP = (real*)(w + 16 + align_up(nb * es, 16));
-        a.VP = (real*)(w + 16 + 2 * align_up(nb * es, 16));
         a.crec = (double*)(w + 16);
     }
     a.xchg_npub = 1;
@@ -245,7 +250,7 @@ template <typename real> int fill_kargs(const MppiFusedParams* p, KArgs<real>& a
     if (!any_peer || a.export_partial) a.world = a.export_partial ? a.world : 1;
     if (p->workspace != nullptr && (a.world == 1 || a.export_partial)) {
         // not sharded in-kernel: the record mailbox is this GPU's own, behind the partials in the workspace
-        a.peers[0] = (unsigned long long*)((unsigned char*)p->workspace + ws_partials_bytes(nb, a.R, es));
+        a.peers[0] = (unsigned long long*)((unsigned char*)p->workspace + ws_partials_bytes(nb, a.R));
         a.xchg_parity_words = MPPI_LL_LOCAL_WORDS;
     }
     return MPPI_OK;

@@ -6,7 +6,7 @@
 //   registers -> bf16 operand tile in shared memory (canonical K-major, no swizzle)
 //   tcgen05.mma.cta_group::1.kind::f16  (one elected thread)  -> fp32 accumulators in TMEM
 //   tcgen05.commit -> mbarrier -> tcgen05.ld of the thread's own row (lane = sample) -> tanh -> next operand row
-// three times per step.  Everything else (sampling, clamp, cost, softmin fold, last-CTA update) is the
+// three times per step.  Everything else (sampling, clamp, cost, the warp-fold softmin and its tail) is the
 // code of mppi_fused.cuh.
 //
 // Round 2: a step is a serial chain of three MMA round trips (7,090 clocks per step measured at BASELINE config 4, the
@@ -228,8 +228,10 @@ __global__ void __launch_bounds__(256, 2) mlp_tc_command_kernel(const __grid_con
     const int tid = threadIdx.x, BD = blockDim.x;      // BD == 256: thread = (sample row tid % 128, half tid / 128)
     const int warp = tid >> 5;
     const int row = tid & 127, half = tid >> 7;
-    const SmemLayout L = make_layout<real>(VARIANT, a.T, NU, a.S, a.R, BD, BD / a.tps, gridDim.x, 0);
+    const SmemLayout L = make_layout<real>(VARIANT, a.T, NU, a.S, a.R, BD, BD / a.tps, fused_layout_nb((int)gridDim.x, 1),
+                                           layout_extra(0, 0, 1, fused_xstage_doubles(a.world > 1 && !a.export_partial, a.world, 1, a.R)));
     Smem<real> sm(smem, L);
+    warp_records_init<real>(a, sm);      // published by the setup barrier below
     const NoiseModel<real>& nm = a.nm;
     const int T = a.T;
     if (a.dbg != nullptr && tid == 32) {
@@ -343,7 +345,6 @@ __global__ void __launch_bounds__(256, 2) mlp_tc_command_kernel(const __grid_con
 
     stage_issue<real, VARIANT, NU>(a, sm);
     bool staged = false;
-    real beta_run = O::inf(), eta_run = (real)0;
 
     // Tile = 128 samples; the two threads of a sample share its draws and its colour/clamp pass (a.tps == 2), thread 0
     // of the pair (half 0, warps 0-3) carries the state and the cost.
@@ -525,9 +526,10 @@ __global__ void __launch_bounds__(256, 2) mlp_tc_command_kernel(const __grid_con
             if (VARIANT == V_SMPPI) c_tot = O::add(c_tot, O::mul(smooth, nm.w_smooth));
             a.cost_total[k] = c_tot;
         }
-        real w_unused;
-        fold_tile<real, VARIANT, false>(a, sm, c_tot, active, nvalid, beta_run, eta_run, w_unused);
+        // the rollout warps (one sample per thread) fold the tile; the rows were ordered by the rollout's barriers
+        if (roller) warp_fold<real, VARIANT, FOLD_ROWS>(a, sm, c_tot, active, nvalid);
         if (tile == blockIdx.x) TC_STAMP(4)     // tile folded
+        if (tile + (int)gridDim.x < a.n_tiles) __syncthreads();      // the tile is refilled by the next pass
     }
     if (!staged) stage_finish<real, VARIANT, NU>(a, sm);
     tc::fence_before();
@@ -536,7 +538,7 @@ __global__ void __launch_bounds__(256, 2) mlp_tc_command_kernel(const __grid_con
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"((uint32_t)TMEM_COLS) : "memory");
     }
     TC_STAMP(5)         // TMEM released
-    publish_and_finish<real, VARIANT, NU>(a, sm, beta_run, eta_run);
+    warp_tail<real, VARIANT, NU>(a, sm);
     if (a.dbg != nullptr && tid == 32) {
         unsigned long long gt;
         asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));

@@ -74,7 +74,6 @@ __device__ void stage_resident(const KArgs<real>& a, Smem<real>& sm) {
         sm.Uraw[j] = __ldcg(a.U + j);
         if (VARIANT == V_SMPPI) sm.Araw[j] = __ldcg(a.A + j);
     }
-    for (int j = tid; j < R; j += BD) sm.Vrun[j] = (real)0;
     if (VARIANT == V_KMPPI) {
         for (int j = tid; j < R; j += BD) sm.thraw[j] = __ldcg(a.theta + j);
         for (int j = tid; j < T * S; j += BD) sm.Ws[j] = a.W[j];            // constants of the controller
@@ -238,7 +237,7 @@ __global__ void __launch_bounds__(640, 1) resident_command_kernel(const __grid_c
         // (5) rollout, fold, tail — the launched kernel's stages
         const real c_tot = split_cost_rollout<Model, real, VARIANT>(a, mp, sm, k, kg, in_range, active);
         if constexpr (STAMPS) stamp(a.dbg, 3);
-        if (tid < BS) warp_fold<real, VARIANT>(a, sm, c_tot, active, nvalid);
+        if (tid < BS) warp_fold<real, VARIANT, VARIANT == V_SMPPI ? FOLD_ROWS2 : FOLD_ROWS>(a, sm, c_tot, active, nvalid);
         if constexpr (STAMPS) stamp(a.dbg, 4);
         const bool finisher = warp_tail<real, VARIANT, NU, true>(a, sm);
         if (finisher) {

@@ -5,7 +5,7 @@ Samples are independent until the softmin, so rank g rolls out the contiguous sl
 index, so the union of all shards is the same sample set for any world size.  Per command each rank
 contributes one record (beta_g, eta_g, V_g[R]) of (2+R) doubles:
 
-* exchange="p2p"  : the fused kernel's last CTA stores the record straight into every peer's mailbox
+* exchange="p2p"  : the kernel's finisher stores the record straight into every peer's mailbox
                     over NVLink (8-byte flagged words, LL style) and spins on its own mailbox — no
                     second launch, no NCCL call on the hot path.
 * exchange="nccl" : the kernel exports the record, `all_gather_into_tensor` moves it, and

@@ -1003,6 +1003,8 @@ class MPPI:
         return self._noise_buf
 
     def _command_stepped(self, state, shift):
+        if self._world > 1:
+            self._check_exchange_status()
         lib = self._lib
         self._ensure_step_buffers()
         if not torch.is_tensor(state):
@@ -1513,11 +1515,9 @@ class MPPI_Batched(MPPI):
         self._Ubuf[:, : self.T * self.nu].copy_(value)
 
     def _variant_pack(self, p):
-        es = _ES[self.dtype]
         rows = self.T * self.nu
         nb_max = min((self.K + 31) // 32 + 1, 148 * 16)
-        stride = (max(16 + 2 * ((nb_max * es + 15) // 16 * 16) + ((nb_max * rows * es + 15) // 16 * 16),
-                      16 + nb_max * (rows + 2) * 8) + 255) // 256 * 256 + 2 * 12288 * 8   # ws_bytes: partials / records + local mailbox
+        stride = (16 + nb_max * (rows + 2) * 8 + 255) // 256 * 256 + 2 * 12288 * 8   # ws_bytes: ticket + records + local mailbox
         self._env_ws_stride = (stride + 255) // 256 * 256
         need = self._env_ws_stride * self.N
         if self._workspace is None or self._workspace.numel() < need:

@@ -2,7 +2,8 @@
 Each rank rolls out its slice; the (beta, eta, V) records are exchanged (a) inside the kernel over
 NVLink peer mailboxes — the cluster records of every rank straight to every peer (direct mode) or one
 combined record per rank —, (b) with an NCCL all-gather + mppi_apply_partials; all must reproduce the
-unsharded update, identically on every rank.  The log of a 2-GPU run is kept under profiles/."""
+unsharded update, identically on every rank — on the fused route, the stepped route (arbitrary callables) and the
+tcgen05 route of the MLP model.  The log of a 2-GPU run is kept under profiles/."""
 import os
 
 import pytest
@@ -100,6 +101,48 @@ def _worker(rank, world, port, out, mode):
             dist.all_gather(lst, many.U.detach().clone().contiguous())
             results[name] = (float((one.U - many.U).abs().max()), worst, all(torch.equal(lst[0], t) for t in lst))
             results[name + f"/records={many.launch_info.xchg_records}/cluster={many.launch_info.cluster_size}"] = (0.0, 0.0, True)
+        # the stepped route (plain callables: no registered model is detected) and the tcgen05 route of the MLP model,
+        # sharded: their softmin tail exchanges one record per rank (in the kernel, or through the library collective)
+        torch.manual_seed(25)
+        mlp = eng.PendulumMLP(torch.nn.Sequential(torch.nn.Linear(3, 32), torch.nn.Tanh(), torch.nn.Linear(32, 32), torch.nn.Tanh(),
+                                                  torch.nn.Linear(32, 2)).to(dev))
+        nav = eng.LinearPoint.toy2d_nav()
+
+        def routed(route, variant, K_, U0, pg, exchange):
+            if route == "tc":        # fp32 with the default tensor_cores: the tcgen05 kernel
+                return eng.MPPI(mlp.dynamics, mlp.running_cost, 2, torch.tensor(1.0), num_samples=K_, horizon=T, device=dev,
+                                u_min=torch.tensor(-2.0), u_max=torch.tensor(2.0), U_init=U0.clone(), process_group=pg,
+                                exchange=exchange, rng_seed=3)
+            dyn, cost = (lambda s, a: nav.dynamics(s, a)), (lambda s, a: nav.running_cost(s, a))
+            kw = dict(num_samples=K_, horizon=T, device=dev, u_max=torch.tensor([1.0, 1.0]), process_group=pg, exchange=exchange,
+                      rng_seed=3)
+            if variant == "mppi":
+                return eng.MPPI(dyn, cost, 2, torch.eye(2), U_init=U0.clone(), **kw)
+            if variant == "smppi":
+                return eng.SMPPI(dyn, cost, 2, torch.eye(2), w_action_seq_cost=5.0, action_max=torch.tensor([1.0, 1.0]), **kw)
+            return eng.KMPPI(dyn, cost, 2, torch.eye(2), U_init=U0.clone(), num_support_pts=5, kernel=eng.RBFKernel(sigma=2), **kw)
+
+        def on_route(c, route):
+            tc = c._model is not None and (c.launch_info.block_threads, c.launch_info.threads_per_sample) == (256, 2)
+            return tc if route == "tc" else c._model is None
+
+        x_of = {"tc": [3.0, 0.5], "stepped": [-3.0, -2.0]}
+        for route, variant in (("stepped", "mppi"), ("stepped", "smppi"), ("stepped", "kmppi"), ("tc", "mppi")):
+            nu_ = 1 if route == "tc" else 2
+            U0 = torch.randn(T, nu_, generator=g) * 0.3
+            z = torch.randn(K, 5 if variant == "kmppi" else T, nu_, generator=g)
+            single = routed(route, variant, K, U0, None, "p2p")
+            single.inject_noise(z)
+            a_ref = single.command(x_of[route]).cpu()
+            for exchange in ("p2p", "nccl"):
+                c = routed(route, variant, K, U0, dist.group.WORLD, exchange)
+                c.inject_noise(z)
+                a = c.command(x_of[route]).cpu()
+                torch.cuda.synchronize()
+                lst = [torch.zeros_like(c.U) for _ in range(world)]
+                dist.all_gather(lst, c.U.detach().clone().contiguous())
+                results[f"{route}/{variant}/{exchange}"] = (float((c.U.cpu() - single.U.cpu()).abs().max()), float((a - a_ref).abs().max()),
+                                                            on_route(c, route) and all(torch.equal(lst[0], t) for t in lst))
         # a nominal drawn at random (no U_init; reset()) is one draw for the whole controller, whatever the ranks' torch seeds
         torch.manual_seed(1000 + rank)
         rnd = eng.MPPI(pend.dynamics, pend.running_cost, 2, torch.tensor(10.0), num_samples=4096, horizon=12, device=dev,
@@ -137,6 +180,25 @@ def _worker(rank, world, port, out, mode):
                     pass
             dist.barrier()
             results["timeout_is_reported"] = (0.0, 0.0, ok)
+            for route in ("stepped", "tc"):
+                nu_ = 1 if route == "tc" else 2
+                lone = routed(route, "mppi", 4096, torch.ones(T, nu_), dist.group.WORLD, "p2p")
+                lone.command(x_of[route])                 # both ranks: fine
+                torch.cuda.synchronize()
+                dist.barrier()
+                ok = on_route(lone, route)
+                if rank == 0:
+                    U_before = lone.U.clone()
+                    a = lone.command(x_of[route], shift_nominal_trajectory=False)     # rank 1 stays away
+                    torch.cuda.synchronize()
+                    ok = ok and bool(torch.equal(lone.U, U_before)) and bool(torch.equal(a.reshape(-1), U_before[0].reshape(-1)))
+                    try:
+                        lone.command(x_of[route])
+                        ok = False
+                    except eng.mppi._cabi.MppiLibraryError:
+                        pass
+                dist.barrier()
+                results[f"timeout_is_reported/{route}"] = (0.0, 0.0, ok)
         out[rank] = results
     finally:
         dist.destroy_process_group()

@@ -306,12 +306,13 @@ def test_fused_reduction_path_matches_oracle(row, split, variant, dtype, monkeyp
         assert info.grid_blocks * tile < K and K % tile < 32
 
 
-# ---- A. the stepped route: softmin_update_kernel -> fold_tile -> publish_and_finish ------------------------------------
-# nb = min(n_tiles, 148 x occupancy, 2368) (plan_geometry); softmin_update_kernel takes 128 registers (ptxas), so
-# occupancy is 65536 / (128 x threads): 8 CTAs of 64 threads, 2 of 256.
-#   nb <= 256        K = 4096: at most 4096 / 64 = 64 tiles at any tile size
-#   256 < nb <= 2 BD K = 80000, 256 threads: 313 tiles, nb = min(313, 148 x 2) = 296 (two passes for some CTAs)
-#   nb > 2 BD        K = 300000, 64 threads: 4688 tiles, nb = min(4688, 148 x 8) = 1184 > 128, partials staged in sS
+# ---- A. the stepped route: softmin_update_kernel -> warp_fold -> warp_tail (no cluster, ticket) -----------------------
+# Every CTA publishes one record; the last arrival combines the grid's nb records from the L2 workspace (combine_global).
+# nb = min(n_tiles, 148 x occupancy, 2368) (plan_geometry); at 109-115 registers (ptxas) the occupancy is 8 CTAs of 64
+# threads, 2 of 256.
+#   few records      K = 4096: at most 4096 / 64 = 64 tiles at any tile size
+#   296 records      K = 80000, 256 threads: 313 tiles, nb = min(313, 148 x 2) = 296 (two passes for some CTAs)
+#   1184 records     K = 300000, 64 threads: 4688 tiles, nb = min(4688, 148 x 8) = 1184, more records than threads
 STEPPED_PATHS = [("nb-le-256", 4096, {}), ("nb-gt-256", 80000, dict(block_threads=256)),
                  ("nb-gt-2BD", 300000, dict(block_threads=64))]
 
@@ -343,21 +344,25 @@ def test_batched_matches_oracle(row, route, dtype):
 # R = T x nu at 31/32/33 and 63/64/65 (pendulum) and 32/64/66 (LinearPoint).  The records path uses 288-sample tiles
 # (9 warp records, 72 per cluster of 8) so that a 66-row fp64 tile and the cluster's records fit in shared memory
 # (about 212 KB; 512-sample tiles would need 300); its 57 tiles round up to 64 CTAs, so the last cluster carries seven
-# CTAs without samples.
+# CTAs without samples.  The one-warp paths run 32-thread CTAs (K = 6000: 188 tiles of 32 > 148 SMs, so no helper threads)
+# that finish in ticket mode: combine_global's column groups must not be wider than the CTA.
 COLUMN_CASES = [("pendulum", T) for T in (31, 32, 33, 63, 64, 65)] + [("linear", T) for T in (16, 32, 33)]
-COLUMN_PATHS = {"fused-narrow": (16384, {}, "c*-narrow-*"), "fused-records": (16384, dict(block_threads=288), "c8-records-*"),
-                "stepped-small": (4096, {}, None), "stepped-large": (64000, dict(block_threads=64), None)}
+_ONE_WARP_TICKET = (("MPPI_B200_CLUSTER", "1"), ("MPPI_B200_XCHG_DIRECT", "0"))
+COLUMN_PATHS = {"fused-narrow": (16384, {}, "c*-narrow-*", ()), "fused-records": (16384, dict(block_threads=288), "c8-records-*", ()),
+                "fused-one-warp": (6000, dict(block_threads=32), "c1-narrow-ticket", _ONE_WARP_TICKET),
+                "stepped-small": (4096, {}, None, ()), "stepped-large": (64000, dict(block_threads=64), None, ()),
+                "stepped-one-warp": (6000, dict(block_threads=32), None, ())}
 
 
 @pytest.mark.parametrize("path", sorted(COLUMN_PATHS))
 @pytest.mark.parametrize("model,T", COLUMN_CASES, ids=[f"{m}-R{T * (1 if m == 'pendulum' else 2)}" for m, T in COLUMN_CASES])
 def test_column_boundaries_match_oracle(model, T, path, monkeypatch):
-    K, ctor, want = COLUMN_PATHS[path]
+    K, ctor, want, env = COLUMN_PATHS[path]
     pb = pendulum() if model == "pendulum" else linear_point()
     if want is None:
         run_parity(pb, "mppi", torch.float64, K, T, route="stepped", seed=T, **ctor)
     else:
-        fused_path_case(monkeypatch, "mppi", torch.float64, K, T, want, pb=pb, **ctor)
+        fused_path_case(monkeypatch, "mppi", torch.float64, K, T, want, env=env, pb=pb, **ctor)
 
 
 # ---- B. wide models -------------------------------------------------------------------------------------------------
